@@ -6,6 +6,7 @@
     python bench.py --impl reference ...                         # CPU arm: the oracle port of the reference path
     python bench.py --workload refiner [--gpus N]                # configs[4]: ProtoRefiner-only sweep, bank cell-sharded over N GPUs
     python bench.py --workload train [--gpus N] [--all-trainable]   # configs[3]: fine-tune step, gradient all-reduce overlapped
+    python bench.py ... --dump-outputs DIR                       # also write the last timed step's outputs as DIR/<name>.npy
 
 One step = one pass of the hot path over one batch of synthetic input:
   infer,   N = 1 : batch 256 four-view panoramas (1024 views), fp16 operands, + head + refine            (configs[1])
@@ -29,6 +30,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the benchmark leaves the source tree as it found it (it may be read-only)
 
 FLOP_PER_VIEW = 381.92e9          # SURVEY.md §8 / BASELINE.md §2 (un-padded, 2*MAC)
 GEMM_FLOP_PER_VIEW = 87.12e9 + 29.04e9 + 232.33e9 + 0.69e9
@@ -138,6 +140,31 @@ class Dist:
             self.dist.destroy_process_group()
 
 
+def host_outputs(name, value, out=None):
+    """Host copies of the tensors in `value` (a tensor or a namedtuple of them, nested; None is skipped), keyed `name`
+    or `name_<field>`."""
+    out = {} if out is None else out
+    if torch.is_tensor(value):
+        out[name] = value.detach().cpu().clone()
+    elif hasattr(value, "_fields"):
+        for f in value._fields:
+            host_outputs(f"{name}_{f}", getattr(value, f), out)
+    return out
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: every array as <directory>/<name>.npy, float64 kept, other floats as float32, integers (indices)
+    as float64, which holds them exactly."""
+    os.makedirs(directory, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.numpy()
+        a = a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in "iub" else np.float32)
+        total += a.nbytes
+        assert total <= 64 << 20, "--dump-outputs: more than 64 MB of outputs"
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def read_profile():
     """Per-launch device times recorded by the library between pg_profile_begin/end: {family: (ms, launches)}."""
     import ctypes as C
@@ -238,6 +265,9 @@ def run_infer(args):
         sampler.start()
     ms, ms_by_rank, res = D.timed(step_device, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:      # the refiner's predictions and SuperGuessr's ModelOutput
+        dump_outputs(args.dump_outputs, host_outputs("refined_preds_LLH", res[0]) |
+                     host_outputs("refined_preds_geocell", res[1]) | host_outputs("model", res[2]))
     e2e_steps = max(2, min(args.steps, 5))
     ms_e2e, e2e_by_rank, _ = D.timed(step_e2e, e2e_steps, 1)
 
@@ -387,6 +417,9 @@ def run_refiner(args):
     ms_f, _, _ = D.timed(only_flush, args.steps, 2)
     ms, ms_by_rank, res = D.timed(step_device, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:      # ProtoRefiner's (loss, preds_LLH, preds_geocell)
+        dump_outputs(args.dump_outputs, host_outputs("loss", res[0]) | host_outputs("preds_LLH", res[1]) |
+                     host_outputs("preds_geocell", res[2]))
     ms_e2e, e2e_by_rank, _ = D.timed(step_e2e, args.steps, 1)
     ms, ms_e2e = ms - ms_f, ms_e2e - ms_f
     lib = _lib.load()
@@ -478,6 +511,13 @@ def run_train(args):
         sampler.start()
     ms, ms_by_rank, loss = D.timed(lambda: step_with(px), args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:      # the step's loss and a fixed sample of every parameter the optimizer updated
+        params = {}
+        for n, p in sg.named_parameters():
+            if p.requires_grad:
+                pick = torch.randperm(p.numel(), generator=torch.Generator().manual_seed(0))[:16384].sort().values
+                params[n] = p.detach().reshape(-1)[pick.to(dev)].cpu()
+        dump_outputs(args.dump_outputs, {"loss": loss.detach().cpu()} | params)
     ms_e2e, _, _ = D.timed(lambda: step_with(px_host.to(dev, non_blocking=True)).cpu(), max(1, min(args.steps, 2)), 1)
     lib = _lib.load()
     lib.pg_profile_begin()
@@ -601,7 +641,7 @@ def run_reference(args):
     threads = best_threads()
     for _ in range(min(args.warmup, 1)):
         cpu_port_images(1, threads)
-    steps = max(1, min(args.steps, 8))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         cpu_port_images(1, threads)
@@ -644,7 +684,10 @@ def main():
     ap.add_argument("--train-batch", type=int, default=128, help="train: four-view samples per GPU per step")
     ap.add_argument("--chunk-views", type=int, default=64)
     ap.add_argument("--all-trainable", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

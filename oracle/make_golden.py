@@ -20,6 +20,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+from oracle import golden  # noqa: E402
 from oracle import reference_shim as rs  # noqa: E402
 from pigeon_b200 import synthetic  # noqa: E402
 from pigeon_b200.vit_engine import VitDims  # noqa: E402
@@ -149,10 +150,9 @@ def train_fixture(tmp):
                     out[f"mt_final_{hn}_w"] = getattr(sg, hn).weight.detach().numpy().copy()
                     out[f"mt_final_{hn}_b"] = getattr(sg, hn).bias.detach().numpy().copy()
             out["centroids"] = sg.lla_geocells.detach().numpy().copy()
-    np.savez_compressed(os.path.join(OUT, "train_head.npz"), emb=emb.numpy(), labels=labels.numpy(),
-                        labels_clf=labels_clf.numpy(), w0=W.numpy(), b0=b.numpy(),
-                        meta=json.dumps(dict(C=C, D=D, B=B, steps=steps, acc=acc, lr=lr, betas=[0.9, 0.999], eps=1e-8,
-                                             weight_decay=0.01)), **out)
+    golden.save("train_head", dict(emb=emb.numpy(), labels=labels.numpy(), labels_clf=labels_clf.numpy(), w0=W.numpy(),
+                                   b0=b.numpy(), **out),
+                dict(C=C, D=D, B=B, steps=steps, acc=acc, lr=lr, betas=[0.9, 0.999], eps=1e-8, weight_decay=0.01, w_seed=71, emb_seed=72))
 
 
 def preprocess_fixture():
@@ -484,13 +484,12 @@ def loops_fixture(tmp):
     arg = np.argsort(saved_idx.flatten()[:n_img])
     consumer = saved.reshape((-1, dims.hidden))[arg]
     out.update(embed_saved=saved, embed_saved_indices=saved_idx, embed_consumer_rows=consumer)
-    np.savez_compressed(os.path.join(OUT, "loops.npz"),
-                        meta=json.dumps(dict(C=C, D=D, N=N, bs=bs, topk=topk, head_seed=91, bank=dict(C=C, P=1500, D=D, members=1.5, seed=90),
-                                             embed=dict(n_img=n_img, bs=ebs, sd_seed=96, px_seed=97, std=0.05, order=order.tolist(),
-                                                        dims=dict(image_size=56, patch_size=14, hidden=256, heads=4, intermediate=512, layers=2)))),
-                        emb=emb.numpy(), labels=labels, labels_clf=labels_clf, cand=cand, head_w=sg.cell_layer.weight.detach().numpy(),
-                        head_b=sg.cell_layer.bias.detach().numpy(), centroids=sg.lla_geocells.detach().numpy(),
-                        **{f"bank_{k}": v for k, v in packed.items()}, **out)
+    golden.save("loops", dict(emb=emb.numpy(), labels=labels, labels_clf=labels_clf, cand=cand,
+                              head_w=sg.cell_layer.weight.detach().numpy(), head_b=sg.cell_layer.bias.detach().numpy(),
+                              centroids=sg.lla_geocells.detach().numpy(), **{f"bank_{k}": v for k, v in packed.items()}, **out),
+                dict(C=C, D=D, N=N, bs=bs, topk=topk, head_seed=91, bank=dict(C=C, P=1500, D=D, members=1.5, seed=90, empty_cells=3),
+                     embed=dict(n_img=n_img, bs=ebs, sd_seed=96, px_seed=97, std=0.05, order=order.tolist(),
+                                dims=dict(image_size=56, patch_size=14, hidden=256, heads=4, intermediate=512, layers=2))))
 
 
 def tower_train_fixtures(tmp):

@@ -202,10 +202,11 @@ def test_evaluate_model_loop_matches_reference_loop_golden(cuda):
     batches of 4 (ragged last batch).  Pins batch order, what is concatenated, what `metrics` receives and the return."""
     from pigeon_b200 import ProtoRefiner, SuperGuessr
     from pigeon_b200.loops import evaluate_model
-    z, meta = load("loops")
+    from oracle import golden
+    z, meta = golden.load("loops")
     N, bs, topk, D = meta["N"], meta["bs"], meta["topk"], meta["D"]
     emb, labels, labels_clf = torch.tensor(z["emb"]), z["labels"], z["labels_clf"]
-    bank = {k[5:]: z[k] for k in z.files if k.startswith("bank_")}
+    bank = {k[5:]: z[k] for k in z if k.startswith("bank_")}
     sg = SuperGuessr(None, panorama=True, num_candidates=topk, embed_dim=D, geocells=z["centroids"])
     with torch.no_grad():
         sg.cell_layer.weight.copy_(torch.tensor(z["head_w"]))
